@@ -19,7 +19,7 @@ The alternative `--partition scout` cuts ONE branch window into chunks seeded by
 (segments.py); measured on this branch it does not work -- a scout loose enough to be cheap leaves the snaking branch
 (profiles/r02_scout_probe.txt, DESIGN.md section 6) -- so it is kept as an option, not the default.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--grid 1024] [--batch 10] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--grid 1024] [--batch 10] [--impl reference] [--dump-outputs DIR]
 
 Besides `e2e` (the plugin surfaces with host vectors) the line carries `e2e_native`: the same window through ONE C-ABI call from and
 to host buffers (bk_palc_run, the PALC loop as host C++ inside the library), with a check that its rows equal the device-resident
@@ -101,6 +101,7 @@ class ClockSampler:
     def stop(self):
         if self.proc:
             self.proc.terminate()
+            self.proc.wait()
         sm = [float(r[0]) for r in self.rows if r and r[0].replace(".", "").isdigit()]
         mx = [float(r[1]) for r in self.rows if len(r) > 1 and r[1].replace(".", "").isdigit()]
         reasons = set()
@@ -301,7 +302,8 @@ class StepTimer:
         def f(st):
             self.stop()
             keep = cb(st) if cb is not None else True
-            self.start()
+            if keep is not False:  # a callback that ends the loop leaves no step to time
+                self.start()
             return keep
         return f
 
@@ -348,19 +350,22 @@ def window_job(bk, ctx, ls, n, u_start, s_total, rank, world, torch, flush, timi
     s0 = ctx.stats()
     torch.cuda.profiler.start()
     info = {"scout_ms": 0.0, "scout_points": 0, "chunk": None, "rejected": 0, "work_newton": 0, "work_linear": 0}
+    # the loop's own bound (step <= max_steps) corrects one step past max_steps and discards it: stop at step `nsteps` instead,
+    # so that the timed window holds exactly the steps the value counts
+    last_step = lambda st: st.step < nsteps
     if spec is not None:
         # --partition speculative: ONE branch on all ranks, rank r correcting with the r-times-halved step (segments.continuation_speculative);
         # spec = (dist, device).  Rows equal the 1-GPU rows; the collectives are an all_gather of 4 doubles and a broadcast of the accepted
         # point per step, both inside the timed region.
         cp1 = cpf()
         cp1.max_steps = nsteps
-        rows, st, sinfo = S.continuation_speculative(P, mkprob(u_start, PAR[0]), alg, cp1, P.norminf, spec[0], torch, spec[1], callback=tm.wrap(None))
+        rows, st, sinfo = S.continuation_speculative(P, mkprob(u_start, PAR[0]), alg, cp1, P.norminf, spec[0], torch, spec[1], callback=tm.wrap(last_step))
         rows = rows[: nsteps + 1]
         info["speculative"] = sinfo
     elif world == 1:
         cp1 = cpf()
         cp1.max_steps = nsteps
-        rows, st = P.continuation(mkprob(u_start, PAR[0]), alg, cp1, normC=P.norminf, callback=tm.wrap(None))
+        rows, st = P.continuation(mkprob(u_start, PAR[0]), alg, cp1, normC=P.norminf, callback=tm.wrap(last_step))
         rows = rows[: nsteps + 1]
     else:
         tm.start()  # the scout's two start-up Newton solves are part of the job
@@ -387,6 +392,7 @@ def window_job(bk, ctx, ls, n, u_start, s_total, rank, world, torch, flush, timi
     s1 = ctx.stats()
     if st is not None:
         info.update(rejected=int(st.nfail), work_newton=int(st.work_newton), work_linear=int(st.work_linear))
+    info["state"] = st
     return rows, ms, {k: s1[k] - s0[k] for k in s1}, info
 
 
@@ -396,6 +402,26 @@ def config_dict(n, workload, K, B):
             "window": f"localized-front branch of examples/SH2d-fronts.jl from lambda = -0.1: {K} batches x {B} continuation steps",
             "batch": B, "newton_tol": 1e-9, "gmres": GMRES, "bls": BLS["kind"], "continuation": CONT,
             "l2": "GPU arm: 256 MiB L2 flush between continuation steps (outside the event pairs); the Krylov basis of a solve exceeds L2"}
+
+
+DUMP_MAX_ENTRIES = 1 << 21  # per state vector (16 MiB in fp64): the dump stays below 64 MiB at any grid
+ROW_KEYS = ("param", "x", "itnewton", "itlinear", "ds", "step", "n_unstable")
+
+
+def dump_outputs(d, rows, st):
+    """Writes what the timed continuation returns to its caller as d/<name>.npy (float64): `branch` = its rows (ROW_KEYS), and
+    the state after its last step: `u`, `p` (solution), `tau_u`, `tau_p` (secant tangent).  A state vector longer than
+    DUMP_MAX_ENTRIES is written as the same seeded sample of entries on every run, so two builds compare entry for entry."""
+    os.makedirs(d, exist_ok=True)
+    host = lambda v: v.numpy() if hasattr(v, "numpy") else np.asarray(v, dtype=np.float64)
+    out = {"branch": np.array([[float(r[k]) for k in ROW_KEYS] for r in rows], dtype=np.float64).reshape(-1, len(ROW_KEYS)),
+           "u": host(st.z_u), "p": np.array([st.z_p]), "tau_u": host(st.tau_u), "tau_p": np.array([st.tau_p])}
+    n = len(out["u"])
+    if n > DUMP_MAX_ENTRIES:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ENTRIES, replace=False))
+        out["u"], out["tau_u"] = out["u"][idx], out["tau_u"][idx]
+    for k, v in out.items():
+        np.save(os.path.join(d, k + ".npy"), np.ascontiguousarray(v, dtype=np.float64))
 
 
 def cpp_opts(cb, max_steps, workers):
@@ -421,7 +447,10 @@ def main():
     ap.add_argument("--branch", default="front", choices=["front", "hexagons"])
     ap.add_argument("--partition", default="replicas", choices=["replicas", "scout", "speculative"],
                     help="N > 1: independent replicas (default), one window cut by a scout, or one branch with speculative step sizes (not measured on GPUs yet)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed window, write its branch rows and final state to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs")
     n, K, B = args.grid, args.steps, args.batch
     BLS["kind"] = args.bls
     BRANCH["kind"] = args.branch
@@ -502,11 +531,17 @@ def main():
     torch.cuda.synchronize()
     sampler.start()
     spec = (dist, f"cuda:{dev}") if (world > 1 and args.partition == "speculative") else None
-    rows, my_ms, delta, info = window_job(bk, ctx, ls, n, u_front, s_total, rank, 1 if spec else jw, torch, flush, nsteps=K * B, spec=spec)
-    torch.cuda.synchronize()
-    if dist:
-        dist.barrier()
-    clocks = sampler.stop()
+    try:
+        rows, my_ms, delta, info = window_job(bk, ctx, ls, n, u_front, s_total, rank, 1 if spec else jw, torch, flush, nsteps=K * B, spec=spec)
+        torch.cuda.synchronize()
+        if dist:
+            dist.barrier()
+    finally:
+        clocks = sampler.stop()
+    if (jw == 1 or spec) and len(rows) != K * B + 1:
+        raise RuntimeError(f"the branch ended after {len(rows) - 1} of the {K * B} continuation steps --steps {K} asks for")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, rows, info["state"])
     tt = torch.tensor([my_ms, float(len(rows)), info["scout_ms"], float(info["rejected"]), float(info["work_newton"]), float(info["work_linear"])],
                       dtype=torch.float64, device=f"cuda:{dev}")
     replica_dev = None
