@@ -8,9 +8,9 @@ palc.py (host-side Newton / newton_palc / continuation loop driving the device k
 """
 from . import lib
 from .lib import (BK200Error, BK_CHAN, BK_SH2D, BK_SH3D, BK_CGL2D, BK_POTRAP_CGL2D, BK_COMPLEX, BK_PC_NONE, BK_PC_SH_DCT,
-                  BK_PC_CHAN_TRIDIAG, BK_PC_CGL_DST, BK_PC_POTRAP_CIRC, build)
+                  BK_PC_CHAN_TRIDIAG, BK_PC_CGL_DST, BK_PC_POTRAP_CIRC, BK_SPARSE, BK_PC_JACOBI, BK_SPARSE_CSR, BK_SPARSE_CSC, build)
 from .core import (Context, DeviceVec, Jacobian, ComplexJacobian, GMRESB200, ComplexGMRESB200, BorderingBLSB200, MatrixFreeBLSB200, ShiftInvertB200,
-                   bls_map, bls_map_block, make_opts, hessenberg_eig)
+                   bls_map, bls_map_block, make_opts, hessenberg_eig, sparse_pattern_args)
 from . import palc
 from . import segments
 from . import floquet

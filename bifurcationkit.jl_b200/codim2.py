@@ -445,6 +445,23 @@ class ComplexProblemB200:
         return self.ctx.cjacobian(x, transpose)
 
 
+class ComplexSparseProblemB200:
+    """Complexified twin of a palc.SparseProblemB200 on a BK_SPARSE | BK_COMPLEX context: the same user J(x, par) (scipy CSR / CSC
+    matrix or pattern values), loaded on the complex context; J(x, p, transpose) -> callable on complex vectors, consumable by
+    ComplexGMRESB200, which sets the transpose flag (J') per call."""
+
+    def __init__(self, cctx, J, params, lens=0, check_pattern=True):
+        assert cctx.complex
+        self.ctx, self.J_, self.params, self.lens, self.check_pattern = cctx, J, list(params), lens, check_pattern
+
+    def J(self, x, p, transpose=False):
+        from .core import ComplexJacobian
+        q = list(self.params)
+        q[self.lens] = p
+        self.ctx.sparse_load(self.J_(_np(x), q), self.check_pattern)
+        return ComplexJacobian(self.ctx, transpose)
+
+
 @dataclass
 class HopfSolution:
     u: object

@@ -163,6 +163,61 @@ class Context:
     def potrap_set_section(self, phi, xpi=None):
         _chk(self, self.lib.bk_potrap_set_section(self.handle, _l.ptr(phi), _l.ptr(xpi)))
 
+    # ---- BK_SPARSE: the Jacobian as a sparse matrix assembled by the caller ----
+    _sp_key = None  # (format, base, indptr, indices) of the pattern loaded last
+    nnz = None
+
+    def sparse_pattern(self, A):
+        """bk_sparse_set_pattern from a scipy CSR / CSC matrix or raw (format, base, ptr, idx) (see sparse_pattern_args)"""
+        fmt, base, nnz, ptr, idx = sparse_pattern_args(A)
+        i64p = C.POINTER(C.c_int64)
+        _chk(self, self.lib.bk_sparse_set_pattern(self.handle, fmt, base, nnz, ptr.ctypes.data_as(i64p), idx.ctypes.data_as(i64p)))
+        self._sp_key, self.nnz = (fmt, base, ptr, idx), nnz
+
+    def sparse_values(self, vals):
+        """bk_sparse_set_values: nnz values in the pattern's order -- a NumPy array, a DeviceVec, or a scipy matrix (its .data)"""
+        assert self.nnz is not None, "sparse_pattern must be called first"
+        if hasattr(vals, "tocsr"):
+            vals = vals.data
+        if not hasattr(vals, "dptr"):
+            vals = np.ascontiguousarray(vals, dtype=np.float64)
+        if len(vals) != self.nnz:
+            raise _l.BK200Error(f"sparse_values: {len(vals)} values for a pattern of {self.nnz} entries")
+        _chk(self, self.lib.bk_sparse_set_values(self.handle, _l.ptr(vals)))
+
+    def sparse_load(self, A, check_pattern=True):
+        """J <- A: a scipy CSR / CSC matrix (its pattern is (re)loaded when it differs from the last one -- compared by indptr /
+        indices unless check_pattern is False, then only when none is loaded yet) or the values array of the loaded pattern"""
+        if hasattr(A, "tocsr"):
+            if self._sp_key is None or (check_pattern and not _same_pattern(self._sp_key, A)):
+                self.sparse_pattern(A)
+        self.sparse_values(A)
+
+
+def sparse_pattern_args(A):
+    """A scipy CSR / CSC matrix, or raw (format, base, ptr, idx) with format BK_SPARSE_CSR / BK_SPARSE_CSC (or "csr" / "csc") and
+    base 0 or 1 (Julia's colptr / rowval as they are: ("csc", 1, colptr, rowval)) -> the arguments (format, base, nnz, ptr, idx) of
+    bk_sparse_set_pattern, ptr and idx as contiguous int64 arrays"""
+    if isinstance(A, tuple):
+        fmt, base, ptr, idx = A
+        fmt = {"csr": _l.BK_SPARSE_CSR, "csc": _l.BK_SPARSE_CSC}.get(fmt, fmt)
+    else:
+        f = getattr(A, "format", None)
+        if f not in ("csr", "csc"):
+            raise _l.BK200Error(f"sparse pattern: a CSR or CSC matrix is needed, got {type(A).__name__} ({f})")
+        fmt, base, ptr, idx = (_l.BK_SPARSE_CSR if f == "csr" else _l.BK_SPARSE_CSC), 0, A.indptr, A.indices
+    if fmt not in (_l.BK_SPARSE_CSR, _l.BK_SPARSE_CSC) or base not in (0, 1):
+        raise _l.BK200Error(f"sparse pattern: bad format {fmt!r} or index base {base!r}")
+    ptr = np.ascontiguousarray(ptr, dtype=np.int64)
+    idx = np.ascontiguousarray(idx, dtype=np.int64)
+    return int(fmt), int(base), int(len(idx)), ptr, idx
+
+
+def _same_pattern(key, A):
+    fmt, base, ptr, idx = key
+    return (base == 0 and fmt == (_l.BK_SPARSE_CSR if A.format == "csr" else _l.BK_SPARSE_CSC)
+            and np.array_equal(ptr, A.indptr) and np.array_equal(idx, A.indices))
+
 
 class DeviceVec:
     """Device-resident fp64 vector with the VectorInterface subset used by the continuation host loop."""

@@ -61,6 +61,28 @@ struct Plan {
 };
 }  // namespace bkg
 
+// BK_SPARSE: one matrix in CSR form (int32 indices) plus the SpMV work partition built with the pattern (bk_sparse.cu)
+struct SpCsr {
+  long long n = 0, nnz = 0;
+  int* rowptr = nullptr;   // n + 1
+  int* col = nullptr;      // nnz
+  double* val = nullptr;   // nnz, CSR order
+  int* perm = nullptr;     // val[k] = src[perm[k]] (src: the caller's value order, or A's CSR values for A'); nullptr: identity
+  int2* blocks = nullptr;  // per CTA: rows [x, y) handled by sub-warps of `width` lanes, or (row, -1): one long row, the whole CTA
+  int nblocks = 0;
+  int width = 32;
+};
+struct SparseMat {
+  long long nnz = 0;
+  SpCsr a;                          // J
+  SpCsr at;                         // J', built at the first transposed application
+  std::vector<int> h_rowptr, h_col; // host copy of J's CSR pattern (source of J')
+  bool have_vals = false;
+  bool at_built = false, at_vals = false;
+  double* stage = nullptr;          // nnz: the caller's values in the caller's order (gather source when a.perm is set)
+  double* diag = nullptr;           // N: diag(J), duplicates summed, 0 where structurally missing
+};
+
 struct Precond {
   int kind = BK_PC_NONE;
   double a0 = 0, a1 = 0;
@@ -82,6 +104,10 @@ struct Precond {
   // potrap circulant preconditioner
   double2* tdft = nullptr;   // exp(-2 pi i j / (M-1))
   double po_r = 0, po_nu = 0, po_T = 0;
+  // Jacobi: out = in / (a0 + a1 diag(J)); the pivots are recomputed (and checked for zeros) at the first application after new values
+  double* jpiv = nullptr;          // a0 + a1 diag(J)
+  unsigned int* jflag = nullptr;
+  bool jdirty = false;
 };
 
 struct bk_ctx {
@@ -141,6 +167,7 @@ struct bk_ctx {
   double* eig_dev = nullptr; // ones (qcap+2) | hcolA (qcap+2) | hcolB (qcap+2) | g (qcap+2) | coef (2*(qcap+2))
   double* eig_pinned = nullptr;
   Precond pc;
+  SparseMat* sp = nullptr;  // BK_SPARSE contexts
   bk_stats stats = {};
   bool timing = false;      // bk_set_timing: event pairs around the fused kernels / preconditioner applications
   int timing_every = 1;     // ... of every timing_every-th bk_gmres call only (event records sit between PDL launches: sampling keeps the overhead small)
@@ -193,6 +220,12 @@ int bk_launch_residual(bk_ctx* c, const double* u_dev, double* out_dev);
 // out = a0*in*in_scale + a1*J*(in*in_scale) [+ bordered terms]; in_scale_ptr (device, may be NULL => 1)
 int bk_launch_apply(bk_ctx* c, const OpDesc& op, const double* in_dev, const double* in_scale_ptr, double* out_dev);
 int bk_potrap_refresh_cache(bk_ctx* c);
+
+// BK_SPARSE (bk_sparse.cu): out = a0 s in + a1 A (s in) on N0 values, A = J or J' (op.transpose)
+int bk_sparse_apply(bk_ctx* c, const OpDesc& op, const double* in_dev, const double* in_scale_ptr, double* out_dev);
+void bk_sparse_free(bk_ctx* c);
+int bk_jacobi_refresh(bk_ctx* c);                                         // pc.jinv from diag(J), pc.a0, pc.a1; zero pivot -> error
+int bk_jacobi_apply(bk_ctx* c, const double* in_dev, double* out_dev);    // N0 values
 
 int bk_precond_apply_dev(bk_ctx* c, const double* in_dev, double* out_dev, long long n);
 void bk_harvest_pc_timing(bk_ctx* c);

@@ -94,12 +94,15 @@ extern "C" int32_t bk_ctx_create(int32_t device, int32_t kind, const int64_t dim
     case BK_SH3D: n = c->dims[0] * c->dims[1] * c->dims[2]; break;
     case BK_CGL2D: n = 2 * c->dims[0] * c->dims[1]; break;
     case BK_POTRAP_CGL2D: n = 2 * c->dims[0] * c->dims[1] * c->dims[2] + 1; break;
+    case BK_SPARSE: n = c->dims[0] * c->dims[1] * c->dims[2]; break;
     default: return bk_fail(c, BK_ERR_ARG, "unknown problem kind", __FILE__, __LINE__);
   }
   BK_CHECK(c, n >= 2, "problem too small");
   BK_CHECK(c, krylov_m >= 1 && krylov_m <= 1024, "krylov_m out of range");
   BK_CHECK(c, !(c->cplx && kind == BK_POTRAP_CGL2D), "BK_COMPLEX is not available for the periodic-orbit functional");
   c->N0 = n;
+  // a sparse context's operator is the loaded matrix, not a linearisation state: bk_sparse_apply reports a missing one
+  c->have_state = (kind == BK_SPARSE);
   if (c->cplx) n *= 2;  // [re; im]
   c->N = n;
   c->m = krylov_m;
@@ -180,6 +183,9 @@ extern "C" int32_t bk_ctx_destroy(bk_ctx* c) {
     cudaEventDestroy(p.second);
   }
   if (c->pc.tdft) cudaFree(c->pc.tdft);
+  if (c->pc.jpiv) cudaFree(c->pc.jpiv);
+  if (c->pc.jflag) cudaFree(c->pc.jflag);
+  bk_sparse_free(c);
   if (c->counters) cudaFree(c->counters);
   for (auto& kv : c->vec_live) cudaFree(kv.first);
   for (double* b : c->stage)

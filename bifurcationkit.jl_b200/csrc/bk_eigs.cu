@@ -19,11 +19,19 @@
 typedef std::complex<double> cplx;
 
 // Eigenvalues of a real upper-Hessenberg matrix (n x n, column-major H[i + j*ldh]) by the complex
-// single-shift QR algorithm with Wilkinson shifts and deflation.
-static bool hess_eigvals(const std::vector<double>& Hr, int n, int ldh, std::vector<cplx>& ev) {
+// single-shift QR algorithm with Wilkinson shifts and deflation.  A subdiagonal entry is neglected when it is below eps
+// times its two diagonal neighbours.  The retry of hess_eigvals for the matrices on which that alone stalls (`robust`):
+// also neglect entries below eps ||H||_F (spectra spread over several decades), and take an isolated trailing 2 x 2 block's
+// eigenvalues from its characteristic polynomial (a double eigenvalue: the shifted QR step cannot shrink the subdiagonal of a
+// block that is a multiple of the identity plus a nilpotent part).
+static bool hess_eigvals_pass(const std::vector<double>& Hr, int n, int ldh, std::vector<cplx>& ev, bool robust) {
   std::vector<cplx> A((size_t)n * n);
   for (int j = 0; j < n; ++j)
     for (int i = 0; i < n; ++i) A[i + (size_t)j * n] = (i <= j + 1) ? cplx(Hr[i + (size_t)j * ldh], 0.0) : cplx(0, 0);
+  double hnorm = 0.0;
+  if (robust)
+    for (const cplx& z : A) hnorm += std::norm(z);
+  hnorm = std::sqrt(hnorm);
   ev.assign(n, cplx(0, 0));
   int hi = n - 1, iter = 0;
   const double eps = 2.2e-16;
@@ -37,7 +45,8 @@ static bool hess_eigvals(const std::vector<double>& Hr, int n, int ldh, std::vec
     while (l > 0) {
       double s = std::abs(A[(l - 1) + (size_t)(l - 1) * n]) + std::abs(A[l + (size_t)l * n]);
       if (s == 0.0) s = 1.0;
-      if (std::abs(A[l + (size_t)(l - 1) * n]) < eps * s) {
+      const double sub = std::abs(A[l + (size_t)(l - 1) * n]);
+      if (sub < eps * s || sub < eps * hnorm) {
         A[l + (size_t)(l - 1) * n] = 0.0;
         break;
       }
@@ -56,6 +65,13 @@ static bool hess_eigvals(const std::vector<double>& Hr, int n, int ldh, std::vec
     cplx tr = a + d, det = a * d - b * c;
     cplx disc = std::sqrt(tr * tr - 4.0 * det);
     cplx m1 = 0.5 * (tr + disc), m2 = 0.5 * (tr - disc);
+    if (robust && l == hi - 1) {  // isolated 2 x 2 block
+      ev[hi - 1] = m1;
+      ev[hi] = m2;
+      hi -= 2;
+      iter = 0;
+      continue;
+    }
     cplx mu = (std::abs(m1 - d) < std::abs(m2 - d)) ? m1 : m2;
     if (iter % 11 == 10) mu += cplx(std::abs(c), 0.37 * std::abs(c));  // exceptional shift
     // QR step on the active block l..hi
@@ -92,6 +108,9 @@ static bool hess_eigvals(const std::vector<double>& Hr, int n, int ldh, std::vec
     for (int i = l; i <= hi; ++i) A[i + (size_t)i * n] += mu;
   }
   return true;
+}
+static bool hess_eigvals(const std::vector<double>& Hr, int n, int ldh, std::vector<cplx>& ev) {
+  return hess_eigvals_pass(Hr, n, ldh, ev, false) || hess_eigvals_pass(Hr, n, ldh, ev, true);
 }
 
 // Eigenvector of the real Hessenberg matrix for eigenvalue theta by inverse iteration (complex LU with

@@ -109,6 +109,8 @@ extern "C" int32_t bk_palc_run(bk_ctx* c, const bk_palc_opts* po, const bk_gmres
   BK_CHECK(c, po && go && u0 && rows && max_rows >= 1, "bk_palc_run: opts, linsolver, u0 and rows are required");
   BK_CHECK(c, po->lens >= 0 && po->lens < BK_MAX_PAR, "bk_palc_run: lens out of range");
   BK_CHECK(c, !c->cplx && c->N == c->N0, "bk_palc_run: real contexts only");
+  BK_CHECK(c, c->kind != BK_SPARSE,
+           "bk_palc_run: a BK_SPARSE context has no residual (F is the caller's function); run the continuation loop on the host");
   BK_CHECK(c, po->newton_maxit >= 1 && po->dsmin > 0 && po->dsmax >= po->dsmin, "bk_palc_run: bad step / Newton limits");
   const long long N = c->N;
   bkpalc::Opts o;

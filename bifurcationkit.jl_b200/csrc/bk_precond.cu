@@ -319,6 +319,9 @@ static int setup_dim(bk_ctx* c, int d, long long n, double inv_h2, int type, boo
   return gen_setup(c, d, (int)n, type);  // always available: unaligned vectors fall back to it
 }
 
+// number of grid dimensions of the DCT preconditioner: SH3d, or a BK_SPARSE context with a 3-D grid shape
+static int pc_ndim(const bk_ctx* c) { return (c->kind == BK_SH3D || (c->kind == BK_SPARSE && c->dims[2] > 1)) ? 3 : 2; }
+
 extern "C" int32_t bk_precond_setup(bk_ctx* c, int32_t kind, double a0, double a1) {
   BK_ENTER(c);
   BK_CUDA(c, cudaStreamSynchronize(c->stream));
@@ -331,14 +334,16 @@ extern "C" int32_t bk_precond_setup(bk_ctx* c, int32_t kind, double a0, double a
   if (!pc.work2) BK_CUDA(c, cudaMalloc(&pc.work2, 8 * (size_t)c->ld));
   const bool even_nx = (c->dims[0] % 2) == 0;
   if (kind == BK_PC_SH_DCT) {
-    BK_CHECK(c, c->kind == BK_SH2D || c->kind == BK_SH3D, "BK_PC_SH_DCT needs a Swift-Hohenberg context");
-    int nd = c->kind == BK_SH3D ? 3 : 2;
+    BK_CHECK(c, c->kind == BK_SH2D || c->kind == BK_SH3D || (c->kind == BK_SPARSE && c->dims[1] > 1),
+             "BK_PC_SH_DCT needs a Swift-Hohenberg context or a grid-shaped BK_SPARSE context");
+    int nd = pc_ndim(c);
     for (int d = 0; d < nd; ++d) {
       double h = 2 * c->lengths[d] / c->dims[d];
       BK_TRY(setup_dim(c, d, c->dims[d], 1.0 / (h * h), 0, even_nx));
     }
   } else if (kind == BK_PC_CGL_DST) {
-    BK_CHECK(c, c->kind == BK_CGL2D || c->kind == BK_POTRAP_CGL2D, "BK_PC_CGL_DST needs a cGL context");
+    BK_CHECK(c, c->kind == BK_CGL2D || c->kind == BK_POTRAP_CGL2D || (c->kind == BK_SPARSE && c->dims[1] > 1),
+             "BK_PC_CGL_DST needs a cGL context or a grid-shaped BK_SPARSE context");
     for (int d = 0; d < 2; ++d) {
       double h = 2 * c->lengths[d] / c->dims[d];
       BK_TRY(setup_dim(c, d, c->dims[d], 1.0 / (h * h), 1, even_nx));
@@ -381,6 +386,15 @@ extern "C" int32_t bk_precond_setup(bk_ctx* c, int32_t kind, double a0, double a
       tri[2 * n + i] = lo[i];
     }
     BK_TRY(upload(c, (void**)&pc.tri, tri.data(), 8 * 3 * n));
+  } else if (kind == BK_PC_JACOBI) {
+    BK_CHECK(c, c->kind == BK_SPARSE, "BK_PC_JACOBI needs a BK_SPARSE context (the kind with an assembled diagonal)");
+    pc.kind = kind;
+    pc.a0 = a0;
+    pc.a1 = a1;
+    pc.jdirty = true;  // no values loaded yet: the pivots are computed (and checked) at the first application
+    const int st = (c->sp && c->sp->have_vals) ? bk_jacobi_refresh(c) : BK_OK;
+    if (st < 0) pc.kind = BK_PC_NONE;
+    return st;
   } else {
     return bk_fail(c, BK_ERR_ARG, "unknown preconditioner kind", __FILE__, __LINE__);
   }
@@ -457,8 +471,8 @@ static int precond_apply_one(bk_ctx* c, const double* in, double* out, long long
   }
   const bool al = aligned16(in, out);
   if (pc.kind == BK_PC_SH_DCT) {
-    const int nx = (int)c->dims[0], ny = (int)c->dims[1], nz = c->kind == BK_SH3D ? (int)c->dims[2] : 1;
-    const int nd = c->kind == BK_SH3D ? 3 : 2;
+    const int nd = pc_ndim(c);
+    const int nx = (int)c->dims[0], ny = (int)c->dims[1], nz = nd == 3 ? (int)c->dims[2] : 1;
     double* A = pc.work;
     double* B = pc.work2;
     const int last = nd - 1;
@@ -506,7 +520,8 @@ static int precond_apply_one(bk_ctx* c, const double* in, double* out, long long
     }
   } else if (pc.kind == BK_PC_CGL_DST) {
     const int nx = (int)c->dims[0], ny = (int)c->dims[1];
-    const long long nblk = (c->kind == BK_POTRAP_CGL2D) ? 2 * c->dims[2] : 2;  // components x slices
+    // components x slices (a grid-shaped BK_SPARSE context: one field per z slice)
+    const long long nblk = (c->kind == BK_POTRAP_CGL2D) ? 2 * c->dims[2] : (c->kind == BK_SPARSE ? c->dims[2] : 2);
     double* A = pc.work;
     double* B = pc.work2;
     BK_TRY(transform_pass(c, 0, 0, in, A, nx, ny, (int)nblk, al));
@@ -536,6 +551,8 @@ static int precond_apply_one(bk_ctx* c, const double* in, double* out, long long
     k_potrap_close<<<(unsigned)((Ns + 255) / 256), 256, 0, c->stream>>>(in, out, Ns, M);
     c->stats.kernel_launches += 2;
     BK_CUDA(c, cudaGetLastError());
+  } else if (pc.kind == BK_PC_JACOBI) {
+    BK_TRY(bk_jacobi_apply(c, in, out));
   } else if (pc.kind == BK_PC_CHAN_TRIDIAG) {
     k_thomas<<<1, 32, 0, c->stream>>>(pc.tri, in, out, (int)N);
     c->stats.kernel_launches++;

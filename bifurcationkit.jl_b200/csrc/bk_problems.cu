@@ -404,6 +404,10 @@ static int launch_kind(bk_ctx* c, const OpDesc& op, const double* in, const doub
                                           c->partials, c->counters + 9);
       break;
     }
+    case BK_SPARSE:
+      BK_TRY(MODE == 1 ? bk_fail(c, BK_ERR_ARG, "BK_SPARSE: F is the caller's function, the context has no residual", __FILE__, __LINE__)
+                       : bk_sparse_apply(c, op, in, sp, out));
+      break;
     default: return bk_fail(c, BK_ERR_ARG, "unknown kind", __FILE__, __LINE__);
   }
   c->stats.kernel_launches++;
@@ -428,7 +432,9 @@ static __global__ void __launch_bounds__(256) k_cshift(double* __restrict__ out,
 }
 
 int bk_launch_apply(bk_ctx* c, const OpDesc& op, const double* in, const double* sp, double* out) {
-  if (op.transpose) BK_CHECK(c, op.kind == BK_SH2D || op.kind == BK_SH3D || op.kind == BK_CGL2D, "J' is not available for this problem kind");
+  if (op.transpose)
+    BK_CHECK(c, op.kind == BK_SH2D || op.kind == BK_SH3D || op.kind == BK_CGL2D || op.kind == BK_SPARSE,
+             "J' is not available for this problem kind");
   if (op.cplx) {
     // ((a0 + i a0i) I + a1 J)(x + i y): the real operator on both halves, then the cross terms of the imaginary shift
     OpDesc half = op;
@@ -470,6 +476,7 @@ int bk_potrap_refresh_cache(bk_ctx* c) {
 extern "C" int32_t bk_residual(bk_ctx* c, const double* u, double* out) {
   BK_ENTER(c);
   BkRange nvtx_range("bk_residual");
+  BK_CHECK(c, c->kind != BK_SPARSE, "bk_residual: a BK_SPARSE context has no residual, F is the caller's function");
   double *du, *dout;
   BK_TRY(bk_stage_in(c, u, c->N0, 0, true, &du));
   BK_TRY(bk_stage_in(c, out, c->N0, 1, false, &dout));
@@ -497,7 +504,8 @@ extern "C" int32_t bk_jac_set_shift_imag(bk_ctx* c, double a0_imag) {
 
 extern "C" int32_t bk_jac_set_transpose(bk_ctx* c, int32_t on) {
   BK_ENTER(c);
-  BK_CHECK(c, !on || c->kind == BK_SH2D || c->kind == BK_SH3D || c->kind == BK_CGL2D, "J' is not available for this problem kind");
+  BK_CHECK(c, !on || c->kind == BK_SH2D || c->kind == BK_SH3D || c->kind == BK_CGL2D || c->kind == BK_SPARSE,
+           "J' is not available for this problem kind");
   c->transpose = on != 0;
   return BK_OK;
 }

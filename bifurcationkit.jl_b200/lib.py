@@ -13,8 +13,11 @@ CSRC = os.path.join(_HERE, "csrc")
 
 BK_OK, BK_NOT_CONVERGED = 0, 1
 BK_CHAN, BK_SH2D, BK_SH3D, BK_CGL2D, BK_POTRAP_CGL2D = 1, 2, 3, 4, 5
+BK_SPARSE = 6  # the Jacobian is a caller-assembled sparse matrix (bk_sparse_set_pattern / bk_sparse_set_values)
 BK_COMPLEX = 0x100  # OR-ed into the kind: complexified context, vectors [re; im]
 BK_PC_NONE, BK_PC_SH_DCT, BK_PC_CHAN_TRIDIAG, BK_PC_CGL_DST, BK_PC_POTRAP_CIRC = 0, 1, 2, 3, 4
+BK_PC_JACOBI = 5
+BK_SPARSE_CSR, BK_SPARSE_CSC = 0, 1
 BK_SIDE_NONE, BK_SIDE_LEFT, BK_SIDE_RIGHT = 0, 1, 2
 BK_ORTH_CGS, BK_ORTH_CGS2 = 0, 1
 
@@ -27,6 +30,7 @@ SYMBOLS = [
     "bk_gmres", "bk_gmres2", "bk_bls_bordering", "bk_bls_matrixfree", "bk_bls_map",
     "bk_bls_block_bordering", "bk_bls_block_matrixfree", "bk_bls_block_map",
     "bk_eigs_shift_invert", "bk_potrap_set_section", "bk_hessenberg_eig", "bk_palc_run",
+    "bk_sparse_set_pattern", "bk_sparse_set_values",
 ]
 
 
@@ -136,6 +140,8 @@ def load():
         "bk_hessenberg_eig": [dp, i32, i32, dp, dp, dp, dp],
         "bk_palc_run": [C.c_void_p, C.POINTER(PalcOpts), C.POINTER(GmresOpts), vp, dbl, vp, dbl, dp, i32, PalcCallback, C.c_void_p,
                         vp, C.POINTER(PalcResult)],
+        "bk_sparse_set_pattern": [C.c_void_p, i32, i32, i64, C.POINTER(i64), C.POINTER(i64)],
+        "bk_sparse_set_values": [C.c_void_p, vp],
     }
     for name, args in sig.items():
         f = getattr(lib, name)

@@ -16,7 +16,7 @@ import numpy as np
 
 from scipy.linalg import blas as _blas
 
-from .core import DeviceVec
+from .core import DeviceVec, Jacobian
 
 SQRT_EPS = math.sqrt(np.finfo(np.float64).eps)  # src/Problems.jl:69
 
@@ -171,6 +171,43 @@ class BifurcationProblemB200:
     def J(self, x, p):
         self._set(p)
         return self.ctx.jacobian(x)
+
+
+def _host(x):
+    """a state as a NumPy array (the user functions of SparseProblemB200 are host code)"""
+    return x.numpy() if isinstance(x, DeviceVec) else x
+
+
+class SparseProblemB200(BifurcationProblemB200):
+    """BifurcationProblem(F, u0, params, lens; J) of a user's own problem on a BK_SPARSE context (examples/brusselator.jl:86-93,
+    J = Jbru_sp): F(x, par) -> residual and J(x, par) -> scipy CSR / CSC matrix (or the values of the pattern already loaded), both
+    host functions of a NumPy state and the parameter list `par` (params with par[lens] = p).  J uploads the values and returns
+    the context's Jacobian, so GMRESB200, the bordered solvers and ShiftInvertB200 run on the device SpMV; the pattern is re-set
+    when it changes (indptr / indices compared on every call unless check_pattern is False, then only the first is loaded)."""
+
+    def __init__(self, ctx, F, J, u0, params, lens=0, record=None, delta=SQRT_EPS, check_pattern=True):
+        super().__init__(ctx, u0, params, lens, record, delta)
+        self.F_, self.J_, self.check_pattern = F, J, check_pattern
+
+    def _par(self, p):
+        q = list(self.params)
+        q[self.lens] = p
+        return q
+
+    def F(self, x, p, out=None):
+        r = np.ascontiguousarray(self.F_(_host(x), self._par(p)), dtype=np.float64)
+        if out is None:
+            return self.ctx.to_device(r) if isinstance(x, DeviceVec) else r
+        if isinstance(out, DeviceVec):
+            out.copyto(self.ctx.to_device(r))
+        else:
+            out[...] = r
+        return out
+
+    def J(self, x, p):
+        self._set(p)
+        self.ctx.sparse_load(self.J_(_host(x), self._par(p)), self.check_pattern)
+        return Jacobian(self.ctx)
 
 
 @dataclass

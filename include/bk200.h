@@ -39,6 +39,12 @@ enum {
   BK_SH3D = 3,   /* examples/SH3d.jl:16-53           params (l, nu)                  dims (Nx,Ny,Nz) */
   BK_CGL2D = 4,  /* examples/cGL2d.jl:6-22,262-318   params (r, mu, nu, c3, c5)      dims (Nx,Ny), N = 2 Nx Ny */
   BK_POTRAP_CGL2D = 5, /* src/periodicorbit/PeriodicOrbitTrapeze.jl:209-330 over BK_CGL2D; dims (Nx,Ny,M), N = 2 Nx Ny M + 1 */
+  /* a Jacobian assembled by the caller as a sparse matrix (J = Jbru_sp, examples/brusselator.jl:50-82; JFmit, examples/
+   * mittleman.jl:56-63; any J supporting mul!, GMRESIterativeSolvers src/LinearSolver.jl:149-206).  dims (N) or a grid
+   * (Nx, Ny[, Nz]) with N = Nx Ny Nz: a grid shape lets BK_PC_SH_DCT / BK_PC_CGL_DST be set up on the context (lengths are only
+   * read by them).  The operator is the matrix of bk_sparse_set_pattern + bk_sparse_set_values; bk_jac_set_state stays legal
+   * (it snapshots u and the parameters) but the operator does not read u.  F is the caller's: bk_residual and bk_palc_run fail. */
+  BK_SPARSE = 6,
   /* OR-ed into one of the kinds above (not BK_POTRAP_CGL2D): a COMPLEXIFIED context for the complex shifts of the Hopf
    * minimally augmented system (src/codim2/MinAugHopf.jl:19-40, shift = Complex(0, -omega)) and complex eigenvector work.
    * Unknowns are z = x + i y stored split, [x; y]: bk_problem_size = 2 N0, with N0 = bk_state_size the size of the real
@@ -56,10 +62,15 @@ enum {
   BK_PC_SH_DCT = 1,     /* (L1 + shift I)^-1 by separable DCT-II (exact for the Neumann-closure operator) */
   BK_PC_CHAN_TRIDIAG = 2, /* lu(P), P = tridiagonal Laplacian with identity boundary rows (chan.jl:108-109) */
   BK_PC_CGL_DST = 3,    /* per-component (a0 I + a1 Lap_dirichlet)^-1 by DST-I (block Jacobi over slices) */
-  BK_PC_POTRAP_CIRC = 4 /* Trapeze PO Jacobian of cGL linearised at the trivial state: DST-I in space (mixed-radix FFT of the odd extension, bk_fft_gen.cuh),
+  BK_PC_POTRAP_CIRC = 4, /* Trapeze PO Jacobian of cGL linearised at the trivial state: DST-I in space (mixed-radix FFT of the odd extension, bk_fft_gen.cuh),
                            u1 +- i u2, DFT over the M-1 cyclic slices, scalar symbol; a0 = period T.  Stand-in for the ILU
                            of the assembled PO Jacobian (examples/cGL2d.jl:209-213) */
+  BK_PC_JACOBI = 5      /* (a0 I + a1 diag(J))^-1 with the current values of a BK_SPARSE context (a structurally missing diagonal
+                           entry counts as 0; a zero pivot is an error at setup, or at the first apply after new values).  The diagonal preconditioner a user
+                           passes as Pl = Diagonal(...) to GMRESIterativeSolvers (src/LinearSolver.jl:149-182) */
 };
+/* sparse pattern formats of bk_sparse_set_pattern: CSC is Julia's SparseMatrixCSC (colptr, rowval) */
+enum { BK_SPARSE_CSR = 0, BK_SPARSE_CSC = 1 };
 enum { BK_SIDE_NONE = 0, BK_SIDE_LEFT = 1, BK_SIDE_RIGHT = 2 };
 enum { BK_ORTH_CGS = 0, BK_ORTH_CGS2 = 1 };
 
@@ -129,8 +140,20 @@ int32_t bk_jvp(bk_ctx* ctx, const double* v, double* out, double a0, double a1);
 /* BK_COMPLEX contexts: imaginary part of the shift a0 of every later operator application (default 0) */
 int32_t bk_jac_set_shift_imag(bk_ctx* ctx, double a0_imag);
 /* apply J' instead of J from now on: apply_jacobian(prob, x, par, dx, true) / jacobian_adjoint (src/codim2/MinAugHopf.jl:79-81,
- * 152-155).  SH2d / SH3d are self-adjoint (no-op), cGL2d transposes its 2 x 2 reaction block; BK_CHAN / BK_POTRAP_CGL2D: error */
+ * 152-155).  SH2d / SH3d are self-adjoint (no-op), cGL2d transposes its 2 x 2 reaction block, BK_SPARSE applies the transposed
+ * matrix; BK_CHAN / BK_POTRAP_CGL2D: error */
 int32_t bk_jac_set_transpose(bk_ctx* ctx, int32_t on);
+
+/* ---- BK_SPARSE contexts: the Jacobian as a caller-assembled sparse matrix (J::SparseMatrixCSC of the examples above; the
+ * linear solvers only need mul!, src/LinearSolver.jl:186-206).
+ *   bk_sparse_set_pattern: format BK_SPARSE_CSR (ptr = row pointers, idx = column indices) or BK_SPARSE_CSC (ptr = colptr,
+ *   idx = rowval, Julia's layout passed unchanged with index_base = 1); HOST arrays, ptr of length N + 1, idx of length nnz.
+ *   Checked: ptr monotone from base to nnz + base, every index in range, N and nnz below 2^31 (else BK_ERR_ARG with a message).
+ *   Duplicate entries are summed (as scipy and SparseArrays do), indices need not be sorted.  Setting a pattern drops the values.
+ *   bk_sparse_set_values: nnz values in the pattern's order, host or device pointer; J is the matrix of the last values given (it
+ *   also refreshes the diagonal of BK_PC_JACOBI).  bk_jac_set_transpose(ctx, 1) applies J' (the adjoint of MinAugHopf.jl:79-81). */
+int32_t bk_sparse_set_pattern(bk_ctx* ctx, int32_t format, int32_t index_base, int64_t nnz, const int64_t* ptr, const int64_t* idx);
+int32_t bk_sparse_set_values(bk_ctx* ctx, const double* vals);
 
 /* ---- K6: preconditioner --------------------------------------------------------------------- */
 int32_t bk_precond_setup(bk_ctx* ctx, int32_t kind, double a0, double a1); /* SH_DCT: (L1 + a0 I)^-1; CGL_DST: (a0 I + a1 Lap)^-1 */

@@ -14,15 +14,19 @@
 #   ls   = BK200.GMRESB200(ctx; reltol = 1e-5, Pr = true)
 #   opts = ContinuationPar(...; newton_options = NewtonPar(linsolver = ls, eigsolver = BK200.ShiftInvertB200(ctx, 0.1, ls)))
 #   br   = continuation(prob, PALC(bls = BK200.BorderingBLSB200(ls)), opts; normC = norminf)
+#
+# A user problem with an assembled sparse Jacobian (examples/brusselator.jl, J = Jbru_sp) runs on a :SPARSE context:
+#   ctx = BK200.Context(:SPARSE, (2n,), (1.0,); krylov_m = 200); BK200.precond!(ctx, :JACOBI, 0.0, 1.0)
+#   ls  = BK200.GMRESB200(ctx; Pl = true)          # methods for J::SparseMatrixCSC load J with BK200.sparse!
 module BK200
 
-using BifurcationKit, LinearAlgebra
+using BifurcationKit, LinearAlgebra, SparseArrays
 const BK = BifurcationKit
 const VI = BK.VI
 const lib = get(ENV, "BK200_LIB", joinpath(@__DIR__, "..", "bifurcationkit.jl_b200", "libbk200.so"))
 
-const KINDS = Dict(:CHAN => 1, :SH2D => 2, :SH3D => 3, :CGL2D => 4, :POTRAP_CGL2D => 5)
-const PCS = Dict(:NONE => 0, :SH_DCT => 1, :CHAN_TRIDIAG => 2, :CGL_DST => 3, :POTRAP_CIRC => 4)
+const KINDS = Dict(:CHAN => 1, :SH2D => 2, :SH3D => 3, :CGL2D => 4, :POTRAP_CGL2D => 5, :SPARSE => 6)
+const PCS = Dict(:NONE => 0, :SH_DCT => 1, :CHAN_TRIDIAG => 2, :CGL_DST => 3, :POTRAP_CIRC => 4, :JACOBI => 5)
 
 struct GmresOpts            # == bk_gmres_opts
     reltol::Cdouble; abstol::Cdouble; restart::Int32; maxiter::Int32
@@ -32,6 +36,7 @@ end
 mutable struct Context
     handle::Ptr{Cvoid}
     N::Int
+    pattern::Any   # :SPARSE contexts: (colptr, rowval) of the pattern loaded last (sparse!)
     # complex = true: BK_COMPLEX context (include/bk200.h) -- vectors [re; im], complex shifts, for MinAugHopf.jl's solves
     function Context(kind::Symbol, dims, lengths; krylov_m = 100, device = 0, complex = false)
         d = Int64[dims..., 1, 1][1:3]; L = Float64[lengths..., 1.0, 1.0][1:3]
@@ -39,7 +44,7 @@ mutable struct Context
         st = ccall((:bk_ctx_create, lib), Int32, (Int32, Int32, Ptr{Int64}, Ptr{Float64}, Int32, Ptr{Ptr{Cvoid}}),
                    device, KINDS[kind] | (complex ? 0x100 : 0), d, L, krylov_m, h)
         st < 0 && error("bk_ctx_create: " * unsafe_string(ccall((:bk_last_error, lib), Cstring, (Ptr{Cvoid},), h[])))
-        c = new(h[], Int(ccall((:bk_problem_size, lib), Int64, (Ptr{Cvoid},), h[])))
+        c = new(h[], Int(ccall((:bk_problem_size, lib), Int64, (Ptr{Cvoid},), h[])), nothing)
         # bk_ctx_destroy frees every vector still alive (vec_live); the handle is nulled so that DeviceVec finalizers
         # running AFTER this one (finalizer order is unspecified for objects that die together) do not touch a freed ctx
         finalizer(c) do x
@@ -130,6 +135,19 @@ function (J::Jac)(dx; a₀ = 0.0, a₁ = 1.0)
     out = like(J.ctx, dx)
     check(J.ctx, ccall((:bk_jvp, lib), Int32, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Float64, Float64), J.ctx.handle, ptr(dx), ptr(out), a₀, a₁))
     out
+end
+
+# ---- :SPARSE contexts: J assembled by the user as a SparseMatrixCSC (J = Jbru_sp, examples/brusselator.jl:50-82) --------------
+"""sparse!(ctx, J): load J on a :SPARSE context and return its `Jac`.  The pattern goes over once, as it is (CSC, 1-based
+colptr / rowval, bk_sparse_set_pattern), and again only when it changes; the values go over on every call."""
+function sparse!(c::Context, J::SparseMatrixCSC{Float64, Int})
+    if c.pattern === nothing || c.pattern[1] != J.colptr || c.pattern[2] != J.rowval
+        check(c, ccall((:bk_sparse_set_pattern, lib), Int32, (Ptr{Cvoid}, Int32, Int32, Int64, Ptr{Int64}, Ptr{Int64}),
+                       c.handle, 1, 1, nnz(J), J.colptr, J.rowval))
+        c.pattern = (copy(J.colptr), copy(J.rowval))
+    end
+    check(c, ccall((:bk_sparse_set_values, lib), Int32, (Ptr{Cvoid}, Ptr{Float64}), c.handle, nonzeros(J)))
+    Jac(c)
 end
 
 # ---- AbstractIterativeLinearSolver (src/LinearSolver.jl:8-12,149-206) --------------------------------------------------
@@ -267,6 +285,18 @@ function (e::ShiftInvertB200)(J::Jac, nev; kwargs...)
                    c.handle, e.sigma, nev, kd, e.tol, e.maxrestart, o, C_NULL, re, im_, vecs, nconv, nops))
     return complex.(re, im_), vecs, nconv[] >= nev, Int(nops[])
 end
+
+# ---- the plugin surfaces for J::SparseMatrixCSC (a :SPARSE context; GMRESIterativeSolvers takes any J with mul!,
+# src/LinearSolver.jl:186-206): load J with sparse! on the solver's context, then the Jac methods above
+(l::GMRESB200)(J::SparseMatrixCSC, rhs; k...) = l(sparse!(l.ctx, J), rhs; k...)
+(l::GMRESB200)(J::SparseMatrixCSC, rhs1, rhs2; k...) = l(sparse!(l.ctx, J), rhs1, rhs2; k...)
+(b::BorderingBLSB200)(J::SparseMatrixCSC, args...; k...) = b(sparse!(b.solver.ctx, J), args...; k...)
+(b::MatrixFreeBLSB200)(J::SparseMatrixCSC, args...; k...) = b(sparse!(b.solver.ctx, J), args...; k...)
+BK.solve_bls_block(lbs::BorderingBLSB200, J::SparseMatrixCSC, a::NTuple{M}, b::NTuple{M}, c::AbstractMatrix, rhst, rhsb; k...) where {M} =
+    BK.solve_bls_block(lbs, sparse!(lbs.solver.ctx, J), a, b, c, rhst, rhsb; k...)
+BK.solve_bls_block(lbs::MatrixFreeBLSB200, J::SparseMatrixCSC, a::NTuple{M}, b::NTuple{M}, c::AbstractMatrix, rhst, rhsb; k...) where {M} =
+    BK.solve_bls_block(lbs, sparse!(lbs.solver.ctx, J), a, b, c, rhst, rhsb; k...)
+(e::ShiftInvertB200)(J::SparseMatrixCSC, nev; k...) = e(sparse!(e.ctx, J), nev; k...)
 
 # ---- the all-native loop (optional): one ccall per BRANCH instead of a dozen per Newton iteration ------------------------
 # bk_palc_run (include/bk200.h) runs continuation(prob, PALC(tangent, bls), opts; normC) of src/Continuation.jl:349-601 for the
